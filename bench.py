@@ -230,6 +230,22 @@ def csr_check(rp, ci, va, row_lo, x_full, y_rows, alpha, nsample=100000, seed=7)
     return float(err.max()) if err.size else 0.0, int(rows.size)
 
 
+DUMP_MAX_ENTRIES = 1 << 22   # 32 MiB of float64 per dumped vector
+
+
+def dump_outputs(directory, vectors):
+    """Writes each float64 torch vector as <directory>/<name>.npy.  A vector longer than DUMP_MAX_ENTRIES is sampled: the
+    entries at DUMP_MAX_ENTRIES distinct indices drawn by a generator seeded with 0, in increasing order, so that two runs
+    of the same workload write the same rows."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, v in vectors.items():
+        if v.numel() > DUMP_MAX_ENTRIES:
+            idx = np.sort(np.random.default_rng(0).choice(v.numel(), DUMP_MAX_ENTRIES, replace=False))
+            v = v[torch.from_numpy(idx).to(v.device)]
+        np.save(os.path.join(directory, name + ".npy"), v.cpu().numpy())
+
+
 # ----------------------------------------------------------------- CPU arm --
 def cpu_reference_run(W, steps, warmup, threads=None, max_nnz=None):
     """The reference's CPU path on this box's host cores, on the same matrix as the GPU arm: CSX with
@@ -301,10 +317,18 @@ def main():
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="N > 1: exchange fused into the SpMV kernel over peer memory (default) or NCCL after it")
     ap.add_argument("--graph-steps", type=int, default=16, help="steps per captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write y of the last timed step as DIR/y.npy (float64; vectors of more than "
+                         "%d entries are sampled on fixed rows), so that two builds can be compared output for output; "
+                         "GPU arm in one process only" % DUMP_MAX_ENTRIES)
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        ap.error("--dump-outputs is implemented for the GPU arm in one process")
     W = workload(args.workload)
 
     if args.impl == "reference":
@@ -504,6 +528,8 @@ def main():
     torch.cuda.synchronize()
     barrier()
     clocks = sampler.finish()
+    if args.dump_outputs:   # one process (checked above): every step, the untimed ones after the timed region too, writes
+        dump_outputs(args.dump_outputs, {"y": y})   # the same y = alpha*A*x from the same x
     ms = float(np.median(region_ms))
     value = 2.0 * nnz * args.steps / (ms * 1e-3) / 1e9
     if peer is not None and peer.error():

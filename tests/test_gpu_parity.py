@@ -726,3 +726,27 @@ def test_blas1_helpers_on_device_vectors():
     api.spx_partition_destroy(part)
     api.spx_mat_destroy(A)
     api.spx_input_destroy(inp)
+
+
+def test_bench_dumps_the_timed_product(tmp_path):
+    """bench.py --dump-outputs writes y = alpha*A*x of the timed path (the whole vector at this size)."""
+    import json
+    import subprocess
+    import sys
+    _torch()
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = str(tmp_path / "dump")
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--workload", "small", "--steps", "4",
+                        "--warmup", "1", "--e2e-steps", "1", "--no-cpu-baseline", "--dump-outputs", out],
+                       capture_output=True, text=True, timeout=900, cwd=root)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+    W = bench.workload("small")
+    rp, ci, va = W.rows(0, W.n)
+    x0 = np.random.default_rng(2).uniform(-1, 1, W.n)   # bench.py's x
+    alpha = line["detail"]["alpha"]
+    y = np.load(os.path.join(out, "y.npy"))
+    assert y.dtype == np.float64 and y.shape == (W.n,)
+    bound = _abs_bound(rp, ci, va, x0, W.n) + 1e-300
+    assert np.max(np.abs(y - alpha * _csr_spmv(rp, ci, va, x0, W.n)) / (abs(alpha) * bound)) <= TOL

@@ -1,8 +1,10 @@
 """The reference's own example programs (src/examples/*.c of SparseX) and its API test program (test/src/sparsex_test.c)
 compile UNCHANGED against include/sparsex/*.h and link against libsparsex_b200.so.  They are compiled from where they lie
-under /root/reference (never copied) into tests/_refex/ (git-ignored; the binaries travel to the GPU box, the sources do
-not), and run there on the GPU — the test program through the reference's own test script (test/scripts/test-sparsex.sh.in
-with its two @...@ placeholders filled in: 13 option sets on the bundled matrices, two inputs that must fail)."""
+in a SparseX source tree (REF below) into tests/_refex/ (git-ignored), and run on the GPU — the test program through the
+reference's own test script (test/scripts/test-sparsex.sh.in with its two @...@ placeholders filled in: 13 option sets on
+the bundled matrices, two inputs that must fail).  These programs are SparseX's own sources, not part of this
+repository, and what they check is their exit status and output as they run against this library, so there is nothing
+to store in their place: without the source tree the tests skip."""
 import os
 import subprocess
 
