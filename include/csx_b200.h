@@ -120,6 +120,35 @@ int csxb_spmv(csxb_matrix_t *m, double alpha, const double *d_x, double beta, do
 int csxb_spmv_host(csxb_matrix_t *m, double alpha, const double *h_x, double beta, double *h_y,
                    int overwrite);
 
+/* ---- transposed product y = alpha * A^T * x (+ beta * y) ----------------------------
+ * What BiCG, QMR, CGLS / LSQR and adjoint solves need next to A*x, without tuning A^T as a second matrix: the
+ * transposed tables list the image y[col] += v * x[row] of every unit under the tiles of its columns and read the
+ * values the forward product reads (set_entry updates reach both; only table bytes are added).
+ *   prepare : builds and uploads the transposed tables (after csxb_upload; idempotent).  The first transposed product
+ *             calls it; call it yourself to keep the set-up out of a timing.  Freed with the matrix.
+ *   spmv_t  : d_x has nrows doubles, d_y ncols doubles.  overwrite as in csxb_spmv: every column of the window
+ *             [CSXB_T_COL_LO, CSXB_T_COL_HI) is written exactly once (0 / beta*y where the column has no entry);
+ *             other columns are not touched.  Asynchronous.  CSX-Sym: A^T = A, runs csxb_spmv (bit-identical).
+ *   spmv_t_host : host buffers, unpipelined (x in, product, the window of y out).  Synchronous.
+ * Partial handles (part_lo..part_hi, csxb_tune_csr_slab): the window is the columns the local partitions read and
+ * y[c] = alpha * (A_local^T x)[c] + beta * y[c] there; summing the partials of all processes is the caller's job (as
+ * for the CSX-Sym halo rows, CSXB_SYM_HALO_LO/HI).
+ * csxb_transpose_info (after prepare, else -1): column window [LO, HI), device bytes of the transposed tables,
+ * algorithmic bytes of one product with overwrite (values + tables read + 8*nrows for x + 8 per window column for y;
+ * add 8 per window column when beta matters), kernels launched per product, heavy columns and their segments (columns
+ * whose many single entries are summed by whole warps), host build time in microseconds.
+ * csxb_decode_coords_t: parity aid; for every device-wide value index (partitions in order, as csxb_decode_coords
+ * numbers them after each partition's value base) the (row, col) of A at which the transposed tables gather it.
+ * A host walk of the host copy of the tables: needs no device and no upload. */
+enum { CSXB_T_COL_LO = 0, CSXB_T_COL_HI = 1, CSXB_T_DEVICE_BYTES = 2, CSXB_T_ALG_BYTES = 3, CSXB_T_LAUNCHES = 4,
+       CSXB_T_HEAVY_COLS = 5, CSXB_T_SEGMENTS = 6, CSXB_T_BUILD_US = 7 };
+int csxb_transpose_prepare(csxb_matrix_t *m);
+int csxb_spmv_t(csxb_matrix_t *m, double alpha, const double *d_x, double beta, double *d_y, int overwrite,
+                void *stream);
+int csxb_spmv_t_host(csxb_matrix_t *m, double alpha, const double *h_x, double beta, double *h_y, int overwrite);
+int64_t csxb_transpose_info(const csxb_matrix_t *m, int what);
+int csxb_decode_coords_t(const csxb_matrix_t *m, int32_t *rows, int32_t *cols);
+
 /* ---- tuned-matrix container, single entries -------------------------------------
  * csxb_save / csxb_load replace SaveTuned / LoadTuned (src/internals/Facade.cpp,
  * CsxSaveRestore.hpp:77-370, a boost::archive) with a Boost-free container of the
@@ -149,6 +178,10 @@ int csxb_group_size(const csxb_group_t *g);
 csxb_matrix_t *csxb_group_member(csxb_group_t *g, int i);
 int csxb_group_device(const csxb_group_t *g, int i);
 int csxb_group_spmv(csxb_group_t *g, double alpha, const double *x, double beta, double *y, int overwrite);
+/* y = alpha*A^T*x (+ beta*y unless overwrite): x has nrows, y ncols entries, same memory kinds as csxb_group_spmv;
+ * synchronous.  Every member computes its partial over its column window; the partials are added in member order on
+ * the first member's device (deterministic).  CSX-Sym: csxb_group_spmv. */
+int csxb_group_spmv_t(csxb_group_t *g, double alpha, const double *x, double beta, double *y, int overwrite);
 int csxb_group_save(csxb_group_t *g, const char *path);
 int csxb_group_get_entry(csxb_group_t *g, int64_t row, int64_t col, double *value);
 int csxb_group_set_entry(csxb_group_t *g, int64_t row, int64_t col, double value);

@@ -80,6 +80,13 @@ void spx_vec_destroy(spx_vector_t *v);
  * side tables, traffic figures. */
 struct csxb_matrix;
 struct csxb_matrix *spx_mat_get_engine(const spx_matrix_t *A);
+/* Transposed product, y = alpha * A^T * x and y = alpha * A^T * x + beta * y: x has nrows and y ncols entries
+ * (SPX_ERR_DIM otherwise).  Same vectors, groups and asynchrony as spx_matvec_mult / spx_matvec_kernel; an
+ * SPX_MAT_REORDER matrix works in the permuted numbering, as they do.  The values are the forward product's, so
+ * spx_mat_set_entry updates reach both. */
+spx_error_t spx_matvec_mult_trans(spx_value_t alpha, const spx_matrix_t *A, const spx_vector_t *x, spx_vector_t *y);
+spx_error_t spx_matvec_kernel_trans(spx_value_t alpha, const spx_matrix_t *A, const spx_vector_t *x, spx_value_t beta,
+                                    spx_vector_t *y);
 /* Block until all SpMVs issued on library vectors have completed. */
 void spx_device_synchronize(void);
 

@@ -624,6 +624,46 @@ spx_error_t spx_matvec_kernel(spx_value_t alpha, const spx_matrix_t *A, const sp
   if (check_spmv_args(A, x, y) != SPX_SUCCESS) return SPX_FAILURE;
   return run_spmv(A, alpha, x, beta, y, 0);
 }
+// y = alpha*A^T*x (+ beta*y): x has nrows, y ncols entries.  Library (managed) vectors on both sides run on the device in
+// place; a plain host buffer on either side goes through the host-buffer path (copies inside the call).
+static spx_error_t run_spmv_t(const spx_matrix_t *Ac, spx_value_t alpha, const spx_vector_t *x, spx_value_t beta,
+                              spx_vector_t *y, int overwrite) {
+  spx_matrix_t *A = const_cast<spx_matrix_t *>(Ac);
+  int rc;
+  if (A->group) {
+    rc = csxb_group_spmv_t(A->group, alpha, x->elements, beta, y->elements, overwrite);
+  } else if (is_managed(x) && is_managed(y)) {
+    const int device = (int)csxb_info(A->csx, CSXB_DEVICE);
+    cudaSetDevice(device);
+    cudaMemPrefetchAsync(x->elements, x->size * 8, device, 0);
+    cudaMemPrefetchAsync(y->elements, y->size * 8, device, 0);
+    rc = csxb_spmv_t(A->csx, alpha, x->elements, beta, y->elements, overwrite, nullptr);
+    if (rc == 0 && !g_async && cudaStreamSynchronize(0) != cudaSuccess) rc = -1;
+  } else {
+    rc = csxb_spmv_t_host(A->csx, alpha, x->elements, beta, y->elements, overwrite);
+  }
+  if (rc != 0) {
+    spx_err_get_handler()(SPX_ERR_TUNED_MAT, __FILE__, __LINE__, __func__, "%s", csxb_last_error());
+    return SPX_FAILURE;
+  }
+  return SPX_SUCCESS;
+}
+static spx_error_t check_spmv_t_args(const spx_matrix_t *A, const spx_vector_t *x, const spx_vector_t *y) {
+  if (!A) { SETERROR_1(SPX_ERR_ARG_INVALID, "invalid matrix handle"); return SPX_FAILURE; }
+  if (!x) { SETERROR_1(SPX_ERR_ARG_INVALID, "invalid vector x"); return SPX_FAILURE; }
+  if (!y) { SETERROR_1(SPX_ERR_ARG_INVALID, "invalid vector y"); return SPX_FAILURE; }
+  if (!check_vec_dim(x, (unsigned long)A->nrows) || !check_vec_dim(y, (unsigned long)A->ncols)) { SETERROR_0(SPX_ERR_DIM); return SPX_FAILURE; }
+  return SPX_SUCCESS;
+}
+spx_error_t spx_matvec_mult_trans(spx_value_t alpha, const spx_matrix_t *A, const spx_vector_t *x, spx_vector_t *y) {
+  if (check_spmv_t_args(A, x, y) != SPX_SUCCESS) return SPX_FAILURE;
+  return run_spmv_t(A, alpha, x, 0.0, y, 1);
+}
+spx_error_t spx_matvec_kernel_trans(spx_value_t alpha, const spx_matrix_t *A, const spx_vector_t *x, spx_value_t beta,
+                                    spx_vector_t *y) {
+  if (check_spmv_t_args(A, x, y) != SPX_SUCCESS) return SPX_FAILURE;
+  return run_spmv_t(A, alpha, x, beta, y, 0);
+}
 spx_error_t spx_matvec_kernel_csr(spx_matrix_t **A, spx_index_t nrows, spx_index_t ncols, const spx_index_t *rowptr,
                                   const spx_index_t *colind, const spx_value_t *values, spx_value_t alpha,
                                   const spx_vector_t *x, spx_value_t beta, spx_vector_t *y) {  // matvec.c:622-673

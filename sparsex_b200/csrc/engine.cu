@@ -21,6 +21,7 @@
 #include <cuda_runtime.h>
 
 #include <chrono>
+#include <memory>
 
 #include <climits>
 #include <cstdio>
@@ -284,6 +285,15 @@ __global__ void __launch_bounds__(256) csx_stream_fixup_kernel(const __grid_cons
   }
 }
 
+// Heavy columns of the transposed product: one warp per segment (gather_kernel.cuh: t_segment_warp).
+__global__ void __launch_bounds__(256) csx_t_segment_kernel(const uint2 *__restrict__ ent, const uint32_t *__restrict__ seg,
+                                                            uint32_t nseg, const double *__restrict__ values,
+                                                            const double *__restrict__ x, double *__restrict__ scratch) {
+  const uint32_t s = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (s >= nseg) return;
+  t_segment_warp(ent, seg, values, x, scratch, s, (int)(threadIdx.x & 31));
+}
+
 // --------------------------------------------------------------- host side --
 static thread_local std::string g_last_error;
 static int fail(const std::string &m) { g_last_error = m; return -1; }
@@ -293,6 +303,16 @@ static int fail(const std::string &m) { g_last_error = m; return -1; }
     if (e_ != cudaSuccess)                                                                     \
       return fail(std::string(#call) + ": " + cudaGetErrorString(e_));                         \
   } while (0)
+
+// Tables of the transposed product on the device (csxb_transpose_prepare); they reference the forward values.
+struct TransState {
+  TransLayout lay;
+  PartDev P;                           // row owner = columns of A; heavy-column fix-up in P.sk_fix_*
+  const uint2 *hent = nullptr;         // heavy-column segments
+  const uint32_t *hseg = nullptr;
+  int64_t dev_bytes = 0, alg_bytes = 0, launches = 0, build_us = 0;
+  double *d_x = nullptr, *d_y = nullptr;   // staging for csxb_spmv_t_host (nrows / ncols doubles)
+};
 
 struct csxb_matrix {
   CsxMatrix host;
@@ -321,6 +341,7 @@ struct csxb_matrix {
   int64_t bytes[7] = {0, 0, 0, 0, 0, 0, 0};
   std::vector<std::string> logs;
   std::vector<RowIndex> row_index;   // per partition, built on the first csxb_get/set_entry
+  std::unique_ptr<TransState> trans;   // csxb_transpose_prepare (its device arrays are in allocs)
   ~csxb_matrix() {
     if (!allocs.empty() || d_x || d_y || s_h2d) {
       int cur = -1;
@@ -1011,6 +1032,165 @@ int csxb_spmv_host(csxb_matrix_t *m, double alpha, const double *h_x, double bet
     }
   }
   if (cur != m->device && cur >= 0) CUDA_TRY(cudaSetDevice(cur));
+  return 0;
+}
+
+// ---- transposed product y = alpha*A^T*x + beta*y (gpu_layout.hpp: TransLayout) ---------------------------------------
+// Runs on the device's current value array, so csxb_set_entry updates reach it with no extra work.  Launches: the heavy
+// column segments (if any), the gather over the transposed tables (writes every column of the window once), the fix-up
+// that adds the segment sums (if any).
+struct DeviceGuard {   // restores the caller's device
+  int d = -1;
+  DeviceGuard() { cudaGetDevice(&d); }
+  ~DeviceGuard() { if (d >= 0) cudaSetDevice(d); }
+};
+
+int csxb_transpose_prepare(csxb_matrix_t *m) {
+  if (!m) return fail("invalid argument");
+  if (m->host.symmetric || m->trans) return 0;
+  if (!m->uploaded) return fail("matrix not uploaded (csxb_upload)");
+  DeviceGuard guard;
+  const auto t0 = std::chrono::steady_clock::now();
+  std::unique_ptr<TransState> T(new TransState);
+  // CSX-Sym is excluded above: partitions own nrows rows, the layout the upload built
+  std::string e = build_transpose_layout(m->host, m->layout, T->lay);
+  if (!e.empty()) return fail("transposed layout: " + e);
+  CUDA_TRY(cudaSetDevice(m->device));
+  const TransLayout &TL = T->lay;
+  const PartLayout &pl = TL.part;
+  PartDev &P = T->P;
+  memset(&P, 0, sizeof(P));
+  KindEntry *kt = nullptr; uint32_t *tx = nullptr; XDesc *xd = nullptr;
+  if (dev_copy(m, TL.ktab.data(), TL.ktab.size(), &kt) || dev_copy(m, pl.tile_xoff.data(), pl.tile_xoff.size(), &tx) ||
+      dev_copy(m, pl.xdesc.data(), pl.xdesc.size(), &xd))
+    return -1;
+  int64_t tables = (int64_t)TL.ktab.size() * 8 + (int64_t)pl.tile_xoff.size() * 4 + (int64_t)pl.xdesc.size() * 16;
+  for (size_t t = 0; t < pl.bt.size(); t++) {
+    const BlockTable &B = pl.bt[t];
+    uint32_t *bp = nullptr; BlockImage *bi = nullptr;
+    if (dev_copy(m, B.ptr.data(), B.ptr.size(), &bp) || dev_copy(m, B.ent.data(), B.ent.size(), &bi)) return -1;
+    P.bt[t] = BtDev{bp, (const uint2 *)bi, (long long)B.j0, B.G, B.nloop, B.sf, B.sl, B.image, (uint32_t)((0x100000000ull + B.G - 1) / B.G)};
+    tables += (int64_t)B.ptr.size() * 4 + (int64_t)B.ent.size() * 8;
+  }
+  P.nbt = (int)pl.bt.size();
+  int launches = pl.nrows ? 1 : 0;
+  if (!pl.sk_fix_rows.empty()) {   // heavy columns: segments, fix-up lists, scratch sums (written once, read once)
+    BlockImage *he = nullptr; uint32_t *hs = nullptr, *fp = nullptr, *fi = nullptr; int32_t *fr = nullptr;
+    if (dev_copy(m, TL.hent.data(), TL.hent.size(), &he) || dev_copy(m, TL.hseg.data(), TL.hseg.size(), &hs) ||
+        dev_copy(m, pl.sk_fix_rows.data(), pl.sk_fix_rows.size(), &fr) || dev_copy(m, pl.sk_fix_ptr.data(), pl.sk_fix_ptr.size(), &fp) ||
+        dev_copy(m, pl.sk_fix_idx.data(), pl.sk_fix_idx.size(), &fi))
+      return -1;
+    void *sc = nullptr;
+    CUDA_TRY(cudaMalloc(&sc, std::max<size_t>(pl.sk_scratch, 2) * 8));
+    m->allocs.push_back(sc);
+    T->hent = (const uint2 *)he; T->hseg = hs;
+    P.sk_scratch = (double *)sc; P.sk_fix_rows = fr; P.sk_fix_ptr = fp; P.sk_fix_idx = fi;
+    P.sk_f0 = 0; P.sk_f1 = (uint32_t)pl.sk_fix_rows.size();
+    tables += (int64_t)TL.hent.size() * 8 + (int64_t)TL.hseg.size() * 4 + (int64_t)pl.sk_fix_rows.size() * 8 +
+              (int64_t)pl.sk_fix_idx.size() * 4 + (int64_t)pl.sk_scratch * 16;
+    launches += 2;
+  }
+  P.values = m->d_values; P.tile_xoff = tx; P.xdesc = (const uint4 *)xd; P.ktab = kt;
+  P.nrows = pl.nrows; P.row_start = pl.row_start; P.rpt = pl.rpt;
+  P.values_end = m->d_values + std::max<uint64_t>(m->layout.total_values, 1);
+  // device bytes of the transposed tables (no values: they are the forward ones)
+  T->dev_bytes = (int64_t)TL.ktab.size() * 8 + (int64_t)pl.tile_xoff.size() * 4 + (int64_t)pl.xdesc.size() * 16 +
+                 (int64_t)TL.hent.size() * 8 + (int64_t)TL.hseg.size() * 4 + (int64_t)pl.sk_fix_rows.size() * 4 +
+                 (int64_t)pl.sk_fix_ptr.size() * 4 + (int64_t)pl.sk_fix_idx.size() * 4 + (int64_t)pl.sk_scratch * 8;
+  for (const BlockTable &B : pl.bt) T->dev_bytes += (int64_t)B.ptr.size() * 4 + (int64_t)B.ent.size() * 8;
+  int64_t xrows = 0;
+  for (const CsxPartition &p : m->host.parts) xrows += p.nrows;
+  T->alg_bytes = m->bytes[CSXB_B_VALUES] + tables + 8 * xrows + 8 * pl.nrows;
+  T->launches = launches;
+  T->build_us = (int64_t)(std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count() * 1e6);
+  m->trans = std::move(T);
+  return 0;
+}
+
+int csxb_spmv_t(csxb_matrix_t *m, double alpha, const double *d_x, double beta, double *d_y, int overwrite, void *stream) {
+  if (m->host.symmetric) return csxb_spmv(m, alpha, d_x, beta, d_y, overwrite, stream);   // A^T = A
+  if (!m->trans && csxb_transpose_prepare(m)) return -1;
+  if (on_matrix_device(m)) return -1;
+  cudaStream_t s = (cudaStream_t)stream;
+  const TransState &T = *m->trans;
+  const PartLayout &pl = T.lay.part;
+  if (!pl.nrows) return 0;
+  const uint32_t nseg = (uint32_t)(T.lay.hseg.size() - 1);
+  if (nseg) csx_t_segment_kernel<<<(nseg + 7) / 8, 256, 0, s>>>(T.hent, T.hseg, nseg, m->d_values, d_x, T.P.sk_scratch);
+  if (T.lay.images) launch_gather<true>(T.P, pl, 0, pl.ntiles, d_x, d_y, alpha, beta, overwrite, s, NoXchg());
+  else launch_gather<false>(T.P, pl, 0, pl.ntiles, d_x, d_y, alpha, beta, overwrite, s, NoXchg());
+  if (nseg) {
+    SkIO io;
+    io.x = d_x; io.y = d_y; io.step = nullptr; io.vec[0] = io.vec[1] = nullptr; io.npush = 0;
+    launch_fixup(T.P, 0, (uint32_t)pl.sk_fix_rows.size(), 0, 0, 0, pl.nrows, io, alpha, beta, overwrite, s);
+  }
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+// Host buffers, unpipelined: x (nrows) in, the product, the column window of y (ncols) out.
+int csxb_spmv_t_host(csxb_matrix_t *m, double alpha, const double *h_x, double beta, double *h_y, int overwrite) {
+  if (m->host.symmetric) return csxb_spmv_host(m, alpha, h_x, beta, h_y, overwrite);
+  if (!m->trans && csxb_transpose_prepare(m)) return -1;
+  DeviceGuard guard;
+  CUDA_TRY(cudaSetDevice(m->device));
+  TransState &T = *m->trans;
+  const int64_t nr = m->host.nrows, lo = T.lay.part.row_start, n = T.lay.part.nrows;
+  if (!T.d_x) {
+    CUDA_TRY(cudaMalloc((void **)&T.d_x, (size_t)std::max<int64_t>(nr, 1) * 8));
+    m->allocs.push_back(T.d_x);
+    CUDA_TRY(cudaMalloc((void **)&T.d_y, (size_t)std::max<int64_t>(m->host.ncols, 1) * 8));
+    m->allocs.push_back(T.d_y);
+  }
+  if (!m->s_run) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&m->s_h2d, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&m->s_run, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&m->s_d2h, cudaStreamNonBlocking));
+  }
+  CUDA_TRY(cudaMemcpyAsync(T.d_x, h_x, (size_t)nr * 8, cudaMemcpyDefault, m->s_run));
+  if (!overwrite && n > 0) CUDA_TRY(cudaMemcpyAsync(T.d_y + lo, h_y + lo, (size_t)n * 8, cudaMemcpyDefault, m->s_run));
+  if (csxb_spmv_t(m, alpha, T.d_x, beta, T.d_y, overwrite, m->s_run)) { cudaStreamSynchronize(m->s_run); return -1; }
+  if (n > 0) CUDA_TRY(cudaMemcpyAsync(h_y + lo, T.d_y + lo, (size_t)n * 8, cudaMemcpyDefault, m->s_run));
+  CUDA_TRY(cudaStreamSynchronize(m->s_run));
+  return 0;
+}
+
+int64_t csxb_transpose_info(const csxb_matrix_t *m, int what) {
+  if (!m || !m->trans) return -1;
+  const TransState &T = *m->trans;
+  switch (what) {
+    case CSXB_T_COL_LO: return T.lay.part.row_start;
+    case CSXB_T_COL_HI: return T.lay.part.row_start + T.lay.part.nrows;
+    case CSXB_T_DEVICE_BYTES: return T.dev_bytes;
+    case CSXB_T_ALG_BYTES: return T.alg_bytes;
+    case CSXB_T_LAUNCHES: return T.launches;
+    case CSXB_T_HEAVY_COLS: return T.lay.heavy_cols;
+    case CSXB_T_SEGMENTS: return (int64_t)T.lay.hseg.size() - 1;
+    case CSXB_T_BUILD_US: return T.build_us;
+  }
+  return -1;
+}
+
+// Host walk of the host copy of the transposed tables; builds them on the host when the matrix has none (no device
+// needed).  rows / cols: one entry per device-wide value index.
+int csxb_decode_coords_t(const csxb_matrix_t *mc, int32_t *rows, int32_t *cols) {
+  csxb_matrix *m = const_cast<csxb_matrix *>(mc);
+  if (!m || !rows || !cols) return fail("invalid argument");
+  if (m->host.symmetric) return fail("CSX-Sym has no transposed tables (A^T = A)");
+  TransLayout local;
+  const TransLayout *TL = m->trans ? &m->trans->lay : nullptr;
+  DeviceLayout fl;
+  if (!TL) {
+    std::string e = build_layout(m->host, fl);
+    if (e.empty()) e = build_transpose_layout(m->host, fl, local);
+    if (!e.empty()) return fail("transposed layout: " + e);
+    TL = &local;
+  }
+  int64_t n = 0;
+  for (const CsxPartition &p : m->host.parts) n += p.nnz;
+  std::fill(rows, rows + n, -1);
+  std::fill(cols, cols + n, -1);
+  decode_transpose_coords(*TL, rows, cols);
   return 0;
 }
 

@@ -361,3 +361,28 @@ __device__ __forceinline__ void spmv_tile(const PartDev &P, const double *__rest
   }
 }
 
+
+// ---- heavy columns of the transposed product (gpu_layout.hpp: TransLayout) -------------------------------------------
+// One warp sums segment s of table-4 entries: the lanes stride the entries (two accumulators, loads of both in flight),
+// the fixed butterfly of warp_sum combines the lanes, so the sum does not depend on timing.  Lane 0 stores it in
+// scratch[s]; csx_stream_fixup_kernel adds the segments of a column to y in segment order.
+__device__ __forceinline__ void t_segment_warp(const uint2 *__restrict__ ent, const uint32_t *__restrict__ seg,
+                                               const double *__restrict__ values, const double *__restrict__ x,
+                                               double *__restrict__ scratch, uint32_t s, int lane) {
+  const uint32_t e0 = __ldg(seg + s), e1 = __ldg(seg + s + 1);
+  double a0 = 0.0, a1 = 0.0;
+  uint32_t e = e0 + (uint32_t)lane;
+  for (; e + 32 < e1; e += 64) {
+    const uint2 b0 = __ldg(ent + e), b1 = __ldg(ent + e + 32);
+    const double v0 = __ldg(values + b0.x), x0 = __ldg(x + (b0.y & ~BT_IMAGE));
+    const double v1 = __ldg(values + b1.x), x1 = __ldg(x + (b1.y & ~BT_IMAGE));
+    a0 += v0 * x0;
+    a1 += v1 * x1;
+  }
+  if (e < e1) {
+    const uint2 b = __ldg(ent + e);
+    a0 += __ldg(values + b.x) * __ldg(x + (b.y & ~BT_IMAGE));
+  }
+  const double a = warp_sum(a0 + a1);
+  if (lane == 0) scratch[s] = a;
+}

@@ -198,6 +198,108 @@ class SkBuilder {
   bool first_ = true;
 };
 
+struct BtEnt { int64_t q; int tab; int64_t grp; BlockImage b; };
+// Block-table shapes (G, nloop, sf, sl, image) of table t (gpu_layout.hpp: BlockTable); false when the table is unused.
+bool block_table_shape(const DeviceLayout &L, int t, BlockTable &T) {
+  if (t == 0) { T.G = L.bc_rows; T.nloop = L.bc_align; T.sf = L.bc_align; T.sl = 1; }
+  else if (t == 1) { T.G = L.bc_align; T.nloop = L.bc_rows; T.sf = 1; T.sl = L.bc_align; T.image = 1; }
+  else if (t == 2) { T.G = L.br_align; T.nloop = L.br_cols; T.sf = 1; T.sl = L.br_align; }
+  else if (t == 3) { T.G = L.br_align ? std::max(L.br_img_cols, 1) : 0; T.nloop = L.br_align; T.sf = L.br_align; T.sl = 1; T.image = 1; }
+  else { T.G = 1; T.nloop = 1; T.sf = 0; T.sl = 0; }
+  if (T.G <= 0) { T.G = 1; return false; }
+  return true;
+}
+// Block tables: counting sort of the entries by (owner, table, group); source order inside a group (deterministic sums).
+void sort_block_tables(const DeviceLayout &shape, std::vector<PartLayout> &parts, const std::vector<BtEnt> &btents) {
+  for (size_t q = 0; q < parts.size(); q++) {
+    PartLayout &L = parts[q];
+    if (!L.nrows) continue;
+    L.bt.resize(BT_MAX);
+    for (int t = 0; t < BT_MAX; t++) {
+      BlockTable &T = L.bt[t];
+      if (!block_table_shape(shape, t, T)) continue;
+      T.j0 = L.row_start / T.G;
+      T.ptr.assign((size_t)((L.row_start + L.nrows - 1) / T.G - T.j0 + 1) + 1, 0);
+    }
+  }
+  for (const BtEnt &e : btents) {
+    BlockTable &T = parts[e.q].bt[e.tab];
+    T.ptr[(size_t)(e.grp - T.j0) + 1]++;
+  }
+  std::vector<std::vector<uint32_t>> at(parts.size() * BT_MAX);
+  for (size_t q = 0; q < parts.size(); q++)
+    for (int t = 0; t < BT_MAX && !parts[q].bt.empty(); t++) {
+      BlockTable &T = parts[q].bt[t];
+      for (size_t j = 1; j < T.ptr.size(); j++) T.ptr[j] += T.ptr[j - 1];
+      if (!T.ptr.empty()) T.ent.resize(T.ptr.back());
+      at[q * BT_MAX + t].assign(T.ptr.begin(), T.ptr.end());
+    }
+  for (const BtEnt &e : btents) {
+    BlockTable &T = parts[e.q].bt[e.tab];
+    T.ent[at[(size_t)e.q * BT_MAX + e.tab][(size_t)(e.grp - T.j0)]++] = e.b;
+  }
+  for (size_t q = 0; q < parts.size(); q++) {   // keep the tables that have entries
+    std::vector<BlockTable> keep;
+    for (BlockTable &T : parts[q].bt) if (!T.ent.empty()) keep.push_back(std::move(T));
+    parts[q].bt.swap(keep);
+  }
+}
+// Descriptors: stable counting sort by (owner, tile).
+std::string distribute_descs(std::vector<PartLayout> &parts, const std::vector<Pending> &pend) {
+  std::vector<std::vector<uint32_t>> cnt(parts.size());
+  for (size_t q = 0; q < parts.size(); q++) cnt[q].assign((size_t)parts[q].ntiles + 1, 0);
+  for (const Pending &e : pend) cnt[e.part][e.tile + 1]++;
+  for (size_t q = 0; q < parts.size(); q++) {
+    PartLayout &L = parts[q];
+    for (int64_t t = 0; t < L.ntiles; t++) cnt[q][t + 1] += cnt[q][t];
+    if (cnt[q][L.ntiles] >= 0x80000000u) return "cross-row unit table too large";
+    L.xdesc.resize(cnt[q][L.ntiles]);
+    for (int64_t t = 0; t <= L.ntiles; t++) L.tile_xoff[t] = cnt[q][t];
+  }
+  std::vector<std::vector<uint32_t>> fill(cnt);
+  for (const Pending &e : pend) {
+    parts[e.part].xdesc[fill[e.part][e.tile]++] = e.d;
+    if (((e.d.meta >> 24) & 0xf) != K_DIAG || !(e.d.meta & XD_DELTA1) || (e.d.meta & XD_TRANSPOSED))
+      parts[e.part].xd_diag1_only = false;
+  }
+  return "";
+}
+
+// ---- images y[col] += v * x[row] of block units in block tables 1 and 3 (CSX-Sym and the transposed product) ---------
+// A block unit of the tables (its shape matches bc_align / br_align) whose image can be listed there: sub-blocks of
+// bc_rows rows starting on the sub-block grid and columns aligned to the group width.
+bool block_image_fits(const DeviceLayout &L, uint32_t kind, int64_t delta, int64_t grow, int64_t start_col) {
+  if (kind == K_BCOL) return delta % L.bc_rows == 0 && grow % L.bc_rows == 0 && start_col % L.bc_align == 0;
+  return delta % L.br_cols == 0 && grow % L.br_align == 0 && (L.br_img_cols <= 1 || start_col % L.br_img_cols == 0);
+}
+// Table 1 takes a block-column unit (one entry per sub-block of bc_rows rows), table 3 a block-row unit (one entry per
+// aligned group of br_img_cols columns), each once per row owner of its columns.  owner_end(g, hi): end of the run of
+// columns [g, hi) that the owner of column g holds, -1 when g has none; put(table, group, entry, first column).
+template <class OwnerEnd, class Put>
+bool block_images(const DeviceLayout &L, uint32_t kind, uint32_t voff, int64_t grow, int64_t start_col, int64_t delta,
+                  OwnerEnd owner_end, Put put) {
+  if (kind == K_BCOL) {
+    const int64_t A = L.bc_align, R0 = L.bc_rows;
+    for (int64_t k = 0; k * R0 < delta; k++)
+      for (int64_t g = start_col; g < start_col + A;) {
+        const int64_t e = owner_end(g, start_col + A);
+        if (e < 0) return false;
+        put(1, g / A, BlockImage{voff + (uint32_t)(k * R0 * A), (uint32_t)(grow + k * R0) | BT_IMAGE}, g);
+        g = e;
+      }
+    return true;
+  }
+  const int64_t A = L.br_align, G = std::max(L.br_img_cols, 1);
+  for (int64_t j = 0; j < delta; j += G)
+    for (int64_t g = start_col + j; g < start_col + j + G;) {   // a group can be cut by an owner boundary
+      const int64_t e = owner_end(g, start_col + j + G);
+      if (e < 0) return false;
+      put(3, g / G, BlockImage{voff + (uint32_t)(j * A), (uint32_t)grow | BT_IMAGE}, g);
+      g = e;
+    }
+  return true;
+}
+
 }  // namespace
 
 std::string build_layout(const CsxMatrix &m, DeviceLayout &out) {
@@ -321,7 +423,6 @@ std::string build_layout(const CsxMatrix &m, DeviceLayout &out) {
     if (getenv("CSXB_NO_BLOCK_TABLES")) out.bc_align = out.bc_rows = out.br_align = out.br_cols = out.br_img_cols = 0;   // tuning aid
   }
   // entries of the block tables (table numbers: gpu_layout.hpp)
-  struct BtEnt { int64_t q; int tab; int64_t grp; BlockImage b; };
   std::vector<BtEnt> btents;
   // CSX-Sym: images of the block units that stay with the stream kernel get descriptors
   struct BlockTmp { XDesc d; uint32_t kind, align, other; int64_t cmin, cmax; };
@@ -534,7 +635,8 @@ std::string build_layout(const CsxMatrix &m, DeviceLayout &out) {
         // block tables: one entry per sub-block under the group of rows it adds to (own rows here, images at the owners
         // of its columns)
         const int64_t grow = cp.row_start + row;
-        const bool fits = kind == K_BCOL ? ((int64_t)delta % out.bc_rows == 0 && grow % out.bc_rows == 0 && (!m.symmetric || start_col % out.bc_align == 0))
+        const bool fits = kind == K_BCOL ? (m.symmetric ? block_image_fits(out, kind, delta, grow, start_col)
+                                                        : ((int64_t)delta % out.bc_rows == 0 && grow % out.bc_rows == 0))
                                          : ((int64_t)delta % out.br_cols == 0 && grow % out.br_align == 0);
         if (!fits) {   // (a block cut by a partition boundary ...): its elements one by one
           for (int k = 0; k < size; k++) {
@@ -547,36 +649,28 @@ std::string build_layout(const CsxMatrix &m, DeviceLayout &out) {
               btents.push_back(BtEnt{q, 4, ec, BlockImage{d.voff + (uint32_t)k, (uint32_t)er | BT_IMAGE}});
             }
           }
-        } else if (kind == K_BCOL) {
-          const int64_t A = out.bc_align, R0 = out.bc_rows;
-          for (int64_t k = 0; k * R0 < (int64_t)delta; k++) {
-            const uint32_t vo = d.voff + (uint32_t)(k * R0 * A);
-            btents.push_back(BtEnt{(int64_t)pi, 0, (grow + k * R0) / R0, BlockImage{vo, (uint32_t)start_col}});
-            if (m.symmetric)
-              for (int64_t g = cmin; g <= cmax;) {   // columns owned by one partition, or cut by a partition boundary
-                const int64_t q = owner_of(g);
-                if (q < 0) return "symmetric update targets a row that is not on this device";
-                btents.push_back(BtEnt{q, 1, g / A, BlockImage{vo, (uint32_t)(grow + k * R0) | BT_IMAGE}});
-                g = std::min(cmax + 1, q_start((size_t)q) + q_rows((size_t)q));
-              }
-          }
         } else {
-          const int64_t A = out.br_align, C0 = out.br_cols;
-          for (int64_t k = 0; k * C0 < (int64_t)delta; k++)
-            btents.push_back(BtEnt{(int64_t)pi, 2, grow / A, BlockImage{d.voff + (uint32_t)(k * C0 * A), (uint32_t)(start_col + k * C0)}});
-          if (m.symmetric && out.br_img_cols > 1 && start_col % out.br_img_cols) {   // columns off the grid: a descriptor
+          if (kind == K_BCOL) {
+            const int64_t A = out.bc_align, R0 = out.bc_rows;
+            for (int64_t k = 0; k * R0 < (int64_t)delta; k++)
+              btents.push_back(BtEnt{(int64_t)pi, 0, (grow + k * R0) / R0, BlockImage{d.voff + (uint32_t)(k * R0 * A), (uint32_t)start_col}});
+          } else {
+            const int64_t A = out.br_align, C0 = out.br_cols;
+            for (int64_t k = 0; k * C0 < (int64_t)delta; k++)
+              btents.push_back(BtEnt{(int64_t)pi, 2, grow / A, BlockImage{d.voff + (uint32_t)(k * C0 * A), (uint32_t)(start_col + k * C0)}});
+          }
+          if (m.symmetric && kind == K_BROW && !block_image_fits(out, kind, delta, grow, start_col)) {   // columns off the grid: a descriptor
             XDesc td = d;
             td.meta |= XD_TRANSPOSED;
             if (!list_rows(td, cmin, cmax, pend)) return "symmetric update targets a row that is not on this device";
-          } else if (m.symmetric) {   // image of a block-row unit: one entry per aligned group of its columns (or per column)
-            const int64_t G = std::max(out.br_img_cols, 1);
-            for (int64_t j = 0; j < (int64_t)delta; j += G)
-              for (int64_t g = start_col + j; g < start_col + j + G;) {   // a group can be cut by a partition boundary
-                const int64_t q = owner_of(g);
-                if (q < 0) return "symmetric update targets a row that is not on this device";
-                btents.push_back(BtEnt{q, 3, g / G, BlockImage{d.voff + (uint32_t)(j * A), (uint32_t)grow | BT_IMAGE}});
-                g = std::min(start_col + j + G, q_start((size_t)q) + q_rows((size_t)q));
-              }
+          } else if (m.symmetric) {   // columns owned by one partition, or cut by a partition boundary
+            auto owner_end = [&](int64_t g, int64_t hi) -> int64_t {
+              const int64_t q = owner_of(g);
+              return q < 0 ? -1 : std::min(hi, q_start((size_t)q) + q_rows((size_t)q));
+            };
+            auto put = [&](int tab, int64_t grp, BlockImage b, int64_t g) { btents.push_back(BtEnt{owner_of(g), tab, grp, b}); };
+            if (!block_images(out, kind, d.voff, grow, start_col, delta, owner_end, put))
+              return "symmetric update targets a row that is not on this device";
           }
         }
       } else {
@@ -638,65 +732,213 @@ std::string build_layout(const CsxMatrix &m, DeviceLayout &out) {
   // CSX-Sym: images of the block units that stayed with the stream kernel
   for (const BlockTmp &b : blocks)
     if (!list_rows(b.d, b.cmin, b.cmax, pend)) return "symmetric update targets a row that is not on this device";
-  // block tables: counting sort of the entries by (owner, table, group); source order inside a group (deterministic sums)
-  if (!btents.empty()) {
-    for (size_t q = 0; q < nq; q++) {
-      PartLayout &L = out.parts[q];
-      if (!L.nrows) continue;
-      L.bt.resize(BT_MAX);
-      for (int t = 0; t < BT_MAX; t++) {
-        BlockTable &T = L.bt[t];
-        if (t == 0) { T.G = out.bc_rows; T.nloop = out.bc_align; T.sf = out.bc_align; T.sl = 1; }
-        else if (t == 1) { T.G = out.bc_align; T.nloop = out.bc_rows; T.sf = 1; T.sl = out.bc_align; T.image = 1; }
-        else if (t == 2) { T.G = out.br_align; T.nloop = out.br_cols; T.sf = 1; T.sl = out.br_align; }
-        else if (t == 3) { T.G = out.br_align ? std::max(out.br_img_cols, 1) : 0; T.nloop = out.br_align; T.sf = out.br_align; T.sl = 1; T.image = 1; }
-        else { T.G = 1; T.nloop = 1; T.sf = 0; T.sl = 0; }
-        if (T.G <= 0) { T.G = 1; continue; }
-        T.j0 = L.row_start / T.G;
-        T.ptr.assign((size_t)((L.row_start + L.nrows - 1) / T.G - T.j0 + 1) + 1, 0);
-      }
-    }
-    for (const BtEnt &e : btents) {
-      BlockTable &T = out.parts[e.q].bt[e.tab];
-      T.ptr[(size_t)(e.grp - T.j0) + 1]++;
-    }
-    std::vector<std::vector<uint32_t>> at(nq * BT_MAX);
-    for (size_t q = 0; q < nq; q++)
-      for (int t = 0; t < BT_MAX && !out.parts[q].bt.empty(); t++) {
-        BlockTable &T = out.parts[q].bt[t];
-        for (size_t j = 1; j < T.ptr.size(); j++) T.ptr[j] += T.ptr[j - 1];
-        if (!T.ptr.empty()) T.ent.resize(T.ptr.back());
-        at[q * BT_MAX + t].assign(T.ptr.begin(), T.ptr.end());
-      }
-    for (const BtEnt &e : btents) {
-      BlockTable &T = out.parts[e.q].bt[e.tab];
-      T.ent[at[(size_t)e.q * BT_MAX + e.tab][(size_t)(e.grp - T.j0)]++] = e.b;
-    }
-    for (size_t q = 0; q < nq; q++) {   // keep the tables that have entries
-      std::vector<BlockTable> keep;
-      for (BlockTable &T : out.parts[q].bt) if (!T.ent.empty()) keep.push_back(std::move(T));
-      out.parts[q].bt.swap(keep);
-    }
-  }
+  // block tables, then the descriptors
+  if (!btents.empty()) sort_block_tables(out, out.parts, btents);
+  return distribute_descs(out.parts, pend);
+}
 
-  // distribute the descriptors: stable counting sort by (owner, tile)
-  std::vector<std::vector<uint32_t>> cnt(nq);
-  for (size_t q = 0; q < nq; q++) cnt[q].assign((size_t)out.parts[q].ntiles + 1, 0);
-  for (const Pending &e : pend) cnt[e.part][e.tile + 1]++;
-  for (size_t q = 0; q < nq; q++) {
-    PartLayout &L = out.parts[q];
-    for (int64_t t = 0; t < L.ntiles; t++) cnt[q][t + 1] += cnt[q][t];
-    if (cnt[q][L.ntiles] >= 0x80000000u) return "cross-row unit table too large";
-    L.xdesc.resize(cnt[q][L.ntiles]);
-    for (int64_t t = 0; t <= L.ntiles; t++) L.tile_xoff[t] = cnt[q][t];
+// ---- transposed product (gpu_layout.hpp: TransLayout) -------------------------------------------------------------
+std::string build_transpose_layout(const CsxMatrix &m, const DeviceLayout &fwd, TransLayout &out) {
+  out = TransLayout();
+  if (m.symmetric) return "CSX-Sym needs no transposed tables (A^T = A)";
+  const size_t np = m.parts.size();
+  if (fwd.parts.size() != np) return "the forward layout does not belong to this matrix";
+  if (const char *v = getenv("CSXB_T_HEAVY")) out.heavy_min = std::max(1, atoi(v));   // tuning aids (DESIGN.md section 3b)
+  if (const char *v = getenv("CSXB_T_SEG")) out.seg_len = std::max(32, atoi(v));
+  // columns the local partitions read (all of them when every partition is local)
+  int64_t clo = INT64_MAX, chi = -1;
+  for (const CsxPartition &p : m.parts) if (p.col_max >= p.col_min) { clo = std::min(clo, p.col_min); chi = std::max(chi, p.col_max); }
+  if ((int)np == m.nparts_total) { clo = 0; chi = m.ncols - 1; }
+  if (chi < clo) { clo = 0; chi = -1; }
+  out.ktab = fwd.ktab;
+  std::map<std::pair<uint32_t, uint32_t>, uint32_t> kindex;
+  for (size_t i = 0; i < out.ktab.size(); i++) kindex.insert(std::make_pair(std::make_pair(out.ktab[i].kind_align, out.ktab[i].delta), (uint32_t)i));
+  auto kind_index = [&](uint32_t kind_align, uint32_t delta) -> int64_t {
+    auto it = kindex.find(std::make_pair(kind_align, delta));
+    if (it == kindex.end()) {
+      if (out.ktab.size() >= 65535) return -1;
+      it = kindex.insert(std::make_pair(std::make_pair(kind_align, delta), (uint32_t)out.ktab.size())).first;
+      out.ktab.push_back(KindEntry{kind_align, delta});
+    }
+    return it->second;
+  };
+  const int64_t k_single = kind_index(K_DIAG, 1);
+  if (k_single < 0) return "too many distinct unit kinds on one device";
+  struct Emit { XDesc d; int64_t lo, hi; };   // a descriptor for the columns [lo, hi]
+  std::vector<Emit> em;
+  std::vector<BtEnt> btents;
+  struct Single { int64_t row, col; uint32_t voff; };
+  std::vector<Single> singles;
+  for (size_t pi = 0; pi < np; pi++) {
+    const CsxPartition &cp = m.parts[pi];
+    KindEntry truetab[64];
+    uint32_t id2k[64];
+    size_t nid = 0;
+    for (; nid < cp.id_map.size() && cp.id_map[nid] != -1; nid++) {
+      if (nid >= 64) return "too many unit kinds";
+      if (!classify(cp.id_map[nid], truetab[nid])) return "unsupported pattern id " + std::to_string(cp.id_map[nid]);
+      const int64_t ki = kind_index(truetab[nid].kind_align, truetab[nid].delta);
+      if (ki < 0) return "too many distinct unit kinds on one device";
+      id2k[nid] = (uint32_t)ki;
+    }
+    const uint64_t vbase = fwd.parts[pi].val_base;
+    const uint8_t *ctl = cp.ctl.data();
+    uint64_t p = 0;
+    const uint64_t end = cp.ctl.size();
+    int64_t row = 0, col = 0, v = 0;
+    singles.clear();
+    while (p < end) {   // the unit grammar of build_layout
+      if (p + 2 > end) return "ctl stream truncated";
+      const uint8_t flags = ctl[p++], size = ctl[p++];
+      if (flags & 0x80) { row += (flags & 0x40) ? (int64_t)get_varint(ctl, p) : 1; col = 0; }
+      if (m.full_colind) { uint32_t c; memcpy(&c, ctl + p, 4); p += 4; col = c; }
+      else col = (int64_t)((uint64_t)col + get_varint(ctl, p));
+      if (row >= cp.nrows) return "ctl stream leaves the partition (row " + std::to_string(row) + ")";
+      const uint32_t id = flags & 0x3f;
+      if (id >= nid) return "ctl stream uses an unmapped unit id";
+      if (size == 0) return "ctl unit of size 0";
+      const uint32_t kind = truetab[id].kind_align & 0xff, align = (truetab[id].kind_align >> 8) & 0xff, delta = truetab[id].delta;
+      const int64_t start_col = col, grow = cp.row_start + row, span = (int64_t)(size - 1) * delta;
+      const uint32_t voff = (uint32_t)(vbase + (uint64_t)v);
+      XDesc d;
+      d.voff = voff;
+      d.meta = id2k[id] | ((uint32_t)size << 16) | (kind << 24) | (delta == 1 ? XD_DELTA1 : 0u);
+      if (kind <= K_DELTA64) {
+        if (p + (uint64_t)(size - 1) * delta > end) return "ctl stream truncated";
+        singles.push_back(Single{grow, col, voff});
+        for (int k = 1; k < size; k++) {
+          uint64_t dd = 0;
+          memcpy(&dd, ctl + p, delta);
+          p += delta;
+          col += (int64_t)dd;
+          singles.push_back(Single{grow, col, voff + (uint32_t)k});
+        }
+      } else if (kind == K_HORIZ) {   // row r, columns c + k*delta -> vertical unit of A^T in column r
+        const int64_t ki = kind_index(K_VERT, delta);
+        if (ki < 0) return "too many distinct unit kinds on one device";
+        d.row = (int32_t)start_col; d.col = (int32_t)grow;
+        d.meta = (uint32_t)ki | ((uint32_t)size << 16) | ((uint32_t)K_VERT << 24) | (delta == 1 ? XD_DELTA1 : 0u);
+        em.push_back(Emit{d, start_col, start_col + span});
+        col += span;
+      } else if (kind == K_DIAG) {    // diagonal (r, c) -> diagonal (c, r), same value order
+        d.row = (int32_t)start_col; d.col = (int32_t)grow;
+        em.push_back(Emit{d, start_col, start_col + span});
+      } else if (kind == K_VERT || kind == K_ADIAG) {   // CSX-Sym image descriptors
+        d.row = (int32_t)grow; d.col = (int32_t)start_col;
+        d.meta |= XD_TRANSPOSED;
+        em.push_back(kind == K_VERT ? Emit{d, start_col, start_col} : Emit{d, start_col - span, start_col});
+      } else {
+        if (size % align || size / align != delta) return "inconsistent block unit";
+        const bool in_table = (kind == K_BCOL && (int)align == fwd.bc_align) || (kind == K_BROW && (int)align == fwd.br_align);
+        if (in_table && block_image_fits(fwd, kind, delta, grow, start_col)) {
+          auto owner_end = [](int64_t, int64_t hi) -> int64_t { return hi; };
+          auto put = [&](int tab, int64_t grp, BlockImage b, int64_t) { btents.push_back(BtEnt{0, tab, grp, b}); };
+          block_images(fwd, kind, voff, grow, start_col, delta, owner_end, put);
+        } else {
+          for (int k = 0; k < size; k++) {
+            const int64_t er = grow + (kind == K_BROW ? k % (int)align : k / (int)align);
+            const int64_t ec = start_col + (kind == K_BROW ? k / (int)align : k % (int)align);
+            singles.push_back(Single{er, ec, voff + (uint32_t)k});
+          }
+        }
+      }
+      v += size;
+    }
+    if (v != cp.nnz) return "ctl stream covers " + std::to_string(v) + " values, expected " + std::to_string(cp.nnz);
+    // single elements: one-element diagonal descriptors when they are a tiny minority of the partition (the rule of
+    // build_layout: a stencil's boundary elements keep the diagonal instantiation), else entries of table 4
+    const bool as_desc = singles.size() <= (size_t)(cp.nnz / 256);
+    for (const Single &sg : singles) {
+      if (sg.col < clo || sg.col > chi) return "unit leaves the column range";
+      if (as_desc) {
+        XDesc e;
+        e.voff = sg.voff; e.row = (int32_t)sg.col; e.col = (int32_t)sg.row;
+        e.meta = (uint32_t)k_single | (1u << 16) | ((uint32_t)K_DIAG << 24) | XD_DELTA1;
+        em.push_back(Emit{e, sg.col, sg.col});
+      } else {
+        btents.push_back(BtEnt{0, 4, sg.col, BlockImage{sg.voff, (uint32_t)sg.row | BT_IMAGE}});
+      }
+    }
   }
-  std::vector<std::vector<uint32_t>> fill(cnt);
-  for (const Pending &e : pend) {
-    out.parts[e.part].xdesc[fill[e.part][e.tile]++] = e.d;
-    if (((e.d.meta >> 24) & 0xf) != K_DIAG || !(e.d.meta & XD_DELTA1) || (e.d.meta & XD_TRANSPOSED))
-      out.parts[e.part].xd_diag1_only = false;
+  std::vector<PartLayout> parts(1);
+  PartLayout &L = parts[0];
+  L.row_start = clo; L.nrows = chi - clo + 1;
+  L.rpt = tile_rpt(L.nrows, m.rows_per_thread, !btents.empty());
+  const int64_t TILE_ROWS = L.tile_rows();
+  L.ntiles = (L.nrows + TILE_ROWS - 1) / TILE_ROWS;
+  L.tile_xoff.assign((size_t)L.ntiles + 1, 0);
+  memset(L.idtab, 0, sizeof(L.idtab));
+  std::vector<Pending> pend;
+  for (const Emit &e : em) {
+    if (e.lo < clo || e.hi > chi) return "unit leaves the column range";
+    for (int64_t t = (e.lo - clo) / TILE_ROWS; t <= (e.hi - clo) / TILE_ROWS; t++) pend.push_back(Pending{0, t, e.d});
+    out.images |= (e.d.meta & XD_TRANSPOSED) != 0;
   }
+  if (!btents.empty()) sort_block_tables(fwd, parts, btents);
+  std::string err = distribute_descs(parts, pend);
+  if (!err.empty()) return err;
+  // heavy columns of table 4: their entries go to warp-sized segments
+  for (size_t ti = 0; ti < L.bt.size(); ti++) {
+    BlockTable &T = L.bt[ti];
+    if (T.G != 1 || T.nloop != 1) continue;
+    std::vector<uint32_t> ptr(1, 0);
+    std::vector<BlockImage> ent;
+    L.sk_fix_ptr.assign(1, 0);
+    for (size_t j = 0; j + 1 < T.ptr.size(); j++) {
+      const uint32_t e0 = T.ptr[j], e1 = T.ptr[j + 1];
+      if (e1 - e0 > (uint32_t)out.heavy_min) {
+        L.sk_fix_rows.push_back((int32_t)(T.j0 + (int64_t)j - L.row_start));
+        for (uint32_t e = e0; e < e1; e += (uint32_t)out.seg_len) {
+          L.sk_fix_idx.push_back((uint32_t)out.hseg.size());
+          out.hseg.push_back((uint32_t)out.hent.size());
+          out.hent.insert(out.hent.end(), T.ent.begin() + e, T.ent.begin() + std::min(e1, e + (uint32_t)out.seg_len));
+        }
+        L.sk_fix_ptr.push_back((uint32_t)L.sk_fix_idx.size());
+      } else {
+        ent.insert(ent.end(), T.ent.begin() + e0, T.ent.begin() + e1);
+      }
+      ptr.push_back((uint32_t)ent.size());
+    }
+    out.hseg.push_back((uint32_t)out.hent.size());
+    out.heavy_cols = (int64_t)L.sk_fix_rows.size();
+    L.sk_scratch = (uint32_t)(out.hseg.size() - 1);
+    T.ptr.swap(ptr);
+    T.ent.swap(ent);
+    if (T.ent.empty()) L.bt.erase(L.bt.begin() + (long)ti);
+    break;
+  }
+  if (out.hseg.empty()) out.hseg.push_back(0);
+  out.part = std::move(L);
   return "";
+}
+
+void decode_transpose_coords(const TransLayout &t, int32_t *rows, int32_t *cols) {
+  const PartLayout &L = t.part;
+  auto put = [&](uint64_t vi, int64_t r, int64_t c) { rows[vi] = (int32_t)r; cols[vi] = (int32_t)c; };
+  for (const XDesc &d : L.xdesc) {   // (a descriptor listed under several tiles is decoded once per tile)
+    const uint32_t kind = (d.meta >> 24) & 0xf, size = (d.meta >> 16) & 0xff;
+    const int64_t delta = (d.meta & XD_DELTA1) ? 1 : t.ktab[d.meta & 0xffff].delta;
+    for (uint32_t k = 0; k < size; k++) {
+      const int64_t s = (int64_t)k * delta;
+      if (!(d.meta & XD_TRANSPOSED))   // unit of A^T: element (row + s, x index) is A(x index, row + s)
+        put(d.voff + k, kind == K_VERT ? d.col : (kind == K_DIAG ? d.col + s : d.col - s), d.row + s);
+      else                             // image of a vertical / anti-diagonal unit of A at (row, col)
+        put(d.voff + k, d.row + s, kind == K_ADIAG ? d.col - s : d.col);
+    }
+  }
+  for (const BlockTable &T : L.bt)
+    for (size_t j = 0; j + 1 < T.ptr.size(); j++)
+      for (uint32_t e = T.ptr[j]; e < T.ptr[j + 1]; e++)
+        for (int64_t i = 0; i < T.G; i++) {   // the columns of the group
+          const int64_t g = (T.j0 + (int64_t)j) * T.G + i;
+          if (g < L.row_start || g >= L.row_start + L.nrows) continue;
+          for (int l = 0; l < T.nloop; l++)
+            put((uint64_t)T.ent[e].voff + (uint64_t)(i * T.sf + l * T.sl), (int64_t)(T.ent[e].other & ~BT_IMAGE) + l, g);
+        }
+  for (size_t i = 0; i < L.sk_fix_rows.size(); i++)
+    for (uint32_t j = L.sk_fix_ptr[i]; j < L.sk_fix_ptr[i + 1]; j++)
+      for (uint32_t e = t.hseg[L.sk_fix_idx[j]]; e < t.hseg[L.sk_fix_idx[j] + 1]; e++)
+        put(t.hent[e].voff, (int64_t)(t.hent[e].other & ~BT_IMAGE), L.row_start + L.sk_fix_rows[i]);
 }
 
 }  // namespace spxb

@@ -182,6 +182,33 @@ struct DeviceLayout {
 
 // Decodes every local partition's ctl stream and fills the tables.
 std::string build_layout(const CsxMatrix &m, DeviceLayout &out);
+
+// ---- transposed product y = alpha*A^T*x + beta*y (non-symmetric matrices) ------------------------------------------
+// One row owner whose "rows" are the columns [row_start, row_start + nrows) of A that the local partitions read.  It holds
+// only images y[col] += v * x[row] of the units and references the device-wide values of the forward layout (no values
+// of its own).  A unit whose transpose is itself a table unit gets a forward descriptor with row and column swapped
+// (diagonal (r, c) -> diagonal (c, r); horizontal run in row r -> vertical unit in column r), so a diagonal stencil runs
+// the same gather instantiation both ways.  Vertical and anti-diagonal units get XD_TRANSPOSED descriptors, block units
+// entries of block tables 1 / 3 (the CSX-Sym images), everything else single entries of table 4 (BT_IMAGE, other = row)
+// — or, when such elements are a tiny minority of their partition, one-element diagonal descriptors.
+// Columns with more than heavy_min entries in table 4 are taken out of it: their entries are cut into segments of
+// seg_len entries, each summed by one warp (csx_t_segment_kernel), and the segment sums are added to y in segment order
+// by the stream kernel's fix-up (part.sk_fix_rows / sk_fix_ptr / sk_fix_idx, scratch slot = segment).
+constexpr int T_HEAVY_MIN = 128;         // chosen on R-MAT scale 22 on the B200 (DESIGN.md section 3b)
+constexpr int T_SEG_LEN = 256;
+struct TransLayout {
+  PartLayout part;
+  std::vector<KindEntry> ktab;           // the forward kind table, plus kinds only the transposed units use
+  bool images = false;                   // some descriptor is an XD_TRANSPOSED image (the gather's CSX-Sym form runs)
+  std::vector<BlockImage> hent;          // table-4 entries of the heavy columns, column by column, in source order
+  std::vector<uint32_t> hseg;            // segments + 1: segment s sums hent[hseg[s] .. hseg[s+1])
+  int64_t heavy_cols = 0;
+  int heavy_min = T_HEAVY_MIN, seg_len = T_SEG_LEN;
+};
+// fwd: the forward layout of the same matrix (value offsets, kind table, block-table shapes).
+std::string build_transpose_layout(const CsxMatrix &m, const DeviceLayout &fwd, TransLayout &out);
+// (row, col) of A for every device-wide value index the transposed tables gather (-1 where none does)
+void decode_transpose_coords(const TransLayout &t, int32_t *rows, int32_t *cols);
 // pattern id (CsxUtil.hpp:58-74, CsxUtil.cpp:27-33) -> kernel kind
 bool classify(long pid, KindEntry &ke);
 

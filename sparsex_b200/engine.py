@@ -63,6 +63,16 @@ def lib():
     L.csxb_spmv_host.argtypes = [vp, dbl, vp, dbl, vp, i32]
     L.csxb_decode_coords.restype = i32
     L.csxb_decode_coords.argtypes = [vp, i32, vp, vp]
+    L.csxb_transpose_prepare.restype = i32
+    L.csxb_transpose_prepare.argtypes = [vp]
+    L.csxb_spmv_t.restype = i32
+    L.csxb_spmv_t.argtypes = [vp, dbl, vp, dbl, vp, i32, vp]
+    L.csxb_spmv_t_host.restype = i32
+    L.csxb_spmv_t_host.argtypes = [vp, dbl, vp, dbl, vp, i32]
+    L.csxb_transpose_info.restype = i64
+    L.csxb_transpose_info.argtypes = [vp, i32]
+    L.csxb_decode_coords_t.restype = i32
+    L.csxb_decode_coords_t.argtypes = [vp, vp, vp]
     L.csxb_save.restype = i32
     L.csxb_save.argtypes = [vp, cp]
     L.csxb_load.restype = vp
@@ -90,6 +100,8 @@ def lib():
     L.csxb_group_device.argtypes = [vp, i32]
     L.csxb_group_spmv.restype = i32
     L.csxb_group_spmv.argtypes = [vp, dbl, vp, dbl, vp, i32]
+    L.csxb_group_spmv_t.restype = i32
+    L.csxb_group_spmv_t.argtypes = [vp, dbl, vp, dbl, vp, i32]
     L.csxb_group_save.restype = i32
     L.csxb_group_save.argtypes = [vp, cp]
     L.csxb_group_get_entry.restype = i32
@@ -262,6 +274,44 @@ class CsxMatrix(object):
             raise EngineError(lib().csxb_last_error().decode())
         return y
 
+    def prepare_transpose(self):
+        """Build and upload the tables of the transposed product (csxb_transpose_prepare); idempotent."""
+        if lib().csxb_transpose_prepare(self._h) != 0:
+            raise EngineError(lib().csxb_last_error().decode())
+        return self
+
+    def spmv_t(self, alpha, x, y, beta=0.0, overwrite=True, stream=None):
+        """y = alpha*A^T*x (+ beta*y): x (nrows) and y (ncols) are torch CUDA float64 tensors."""
+        import torch
+        assert x.is_cuda and y.is_cuda and x.dtype == torch.float64 and y.dtype == torch.float64
+        assert x.numel() == self.nrows and y.numel() == self.ncols and x.is_contiguous() and y.is_contiguous()
+        s = torch.cuda.current_stream().cuda_stream if stream is None else stream
+        if lib().csxb_spmv_t(self._h, alpha, x.data_ptr(), beta, y.data_ptr(), int(overwrite), s) != 0:
+            raise EngineError(lib().csxb_last_error().decode())
+        return y
+
+    def spmv_t_host(self, alpha, x, y, beta=0.0, overwrite=True):
+        """y = alpha*A^T*x (+ beta*y) on numpy float64 host arrays (x: nrows, y: ncols)."""
+        assert x.dtype == np.float64 and y.dtype == np.float64 and x.flags.c_contiguous and y.flags.c_contiguous
+        assert x.size == self.nrows and y.size == self.ncols
+        if lib().csxb_spmv_t_host(self._h, alpha, x.ctypes.data, beta, y.ctypes.data, int(overwrite)) != 0:
+            raise EngineError(lib().csxb_last_error().decode())
+        return y
+
+    def transpose_info(self):
+        """csxb_transpose_info after prepare_transpose(): column window, bytes, launches, heavy columns, build time."""
+        keys = ["col_lo", "col_hi", "device_bytes", "alg_bytes", "launches", "heavy_cols", "segments", "build_us"]
+        return {k: lib().csxb_transpose_info(self._h, i) for i, k in enumerate(keys)}
+
+    def decode_coords_t(self):
+        """(rows, cols) of A for every device-wide value index, as the transposed tables gather it (host only)."""
+        n = sum(lib().csxb_part_info(self._h, p, 0) for p in range(self.nparts))
+        r = np.empty(n, np.int32)
+        c = np.empty(n, np.int32)
+        if lib().csxb_decode_coords_t(self._h, r.ctypes.data, c.ctypes.data) != 0:
+            raise EngineError(lib().csxb_last_error().decode())
+        return r, c
+
     def save(self, path):
         if lib().csxb_save(self._h, path.encode()) != 0:
             raise EngineError(lib().csxb_last_error().decode())
@@ -308,6 +358,15 @@ class CsxMatrix(object):
             pass
 
 
+def _vec_ptr(v, n):
+    """numpy float64 array (host buffer) or torch float64 tensor (device or pinned memory) of n entries."""
+    if isinstance(v, np.ndarray):
+        assert v.dtype == np.float64 and v.flags.c_contiguous and v.size == n
+        return v.ctypes.data
+    assert v.is_contiguous() and v.numel() == n
+    return v.data_ptr()
+
+
 class DeviceGroup(object):
     """csxb_group_* (include/csx_b200.h): the partitions of one tuned matrix spread over several GPUs of this process.
     Consumes `matrix` (which must hold all partitions and must not be uploaded)."""
@@ -327,13 +386,13 @@ class DeviceGroup(object):
 
     def spmv(self, alpha, x, y, beta=0.0, overwrite=True):
         """x, y: numpy float64 arrays (host buffers) or torch float64 tensors (device or pinned memory)."""
-        def ptr(v, n):
-            if isinstance(v, np.ndarray):
-                assert v.dtype == np.float64 and v.flags.c_contiguous and v.size == n
-                return v.ctypes.data
-            assert v.is_contiguous() and v.numel() == n
-            return v.data_ptr()
-        if lib().csxb_group_spmv(self._h, alpha, ptr(x, self.ncols), beta, ptr(y, self.nrows), int(overwrite)) != 0:
+        if lib().csxb_group_spmv(self._h, alpha, _vec_ptr(x, self.ncols), beta, _vec_ptr(y, self.nrows), int(overwrite)) != 0:
+            raise EngineError(lib().csxb_last_error().decode())
+        return y
+
+    def spmv_t(self, alpha, x, y, beta=0.0, overwrite=True):
+        """y = alpha*A^T*x (+ beta*y): x has nrows, y ncols entries; the memory kinds of spmv()."""
+        if lib().csxb_group_spmv_t(self._h, alpha, _vec_ptr(x, self.nrows), beta, _vec_ptr(y, self.ncols), int(overwrite)) != 0:
             raise EngineError(lib().csxb_last_error().decode())
         return y
 
@@ -484,6 +543,8 @@ class SpxApi(object):
             "spx_vec_destroy": (None, [VP]),
             "spx_matvec_mult": (i32, [dbl, vp, VP, VP]),
             "spx_matvec_kernel": (i32, [dbl, vp, VP, dbl, VP]),
+            "spx_matvec_mult_trans": (i32, [dbl, vp, VP, VP]),
+            "spx_matvec_kernel_trans": (i32, [dbl, vp, VP, dbl, VP]),
             "spx_matvec_kernel_csr": (i32, [C.POINTER(vp), i32, i32, vp, vp, vp, dbl, VP, dbl, VP]),
             "spx_device_synchronize": (None, []),
             "spx_err_set_handler": (None, [vp]),
